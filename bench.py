@@ -5,6 +5,7 @@
     python bench.py --impl reference --gpus N --steps K --warmup W      # the reference's CPU PyTorch path (oracle port)
     python bench.py --workload multitask --gpus 8                       # configs[2]: B = 512 global, VQA / NLVR2 / RefCOCO thirds
     python bench.py --workload retrieval --gpus 8 --steps 1             # configs[3]: 1000 x 1000 caption-image score matrix
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR    # + the last timed step's outputs as DIR/<name>.npy
 
 A "step" is one forward of one batch of `--batch` pairs per GPU (vqa, multitask: batches shard over ranks with no collective,
 SURVEY.md 8e -> weak scaling) or one whole score matrix (retrieval: captions shard over ranks, ONE NCCL all-gather of the score
@@ -61,7 +62,13 @@ def parse():
     p.add_argument("--captions", type=int, default=1000, help="retrieval: captions (rows of the score matrix)")
     p.add_argument("--images", type=int, default=1000, help="retrieval: images (columns)")
     p.add_argument("--no-reuse", action="store_true", help="retrieval: full forward per pair instead of cached prefixes")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", default="", metavar="DIR",
+                   help="after the timed steps, write what the timed path returned in its last step (rank 0's share) as "
+                        "DIR/<name>.npy, float32, at most 64 MB in all")
+    a = p.parse_args()
+    if a.dump_outputs and a.impl == "reference":
+        p.error("--dump-outputs records the GPU path's outputs; --impl reference has none")
+    return a
 
 
 def env_rank():
@@ -76,6 +83,33 @@ def peaks():
                 "hbm": d["hbm_gbs"], "src": "measured"}
     except Exception:
         return {"bf16_burst": 1590.0, "bf16_sustained": 1400.0, "hbm": 6650.0, "src": "fallback"}
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: each tensor of `arrays` (name -> tensor) as out_dir/<name>.npy in float32.  When they add up to more than
+    DUMP_BYTES, every array keeps the same share of its rows, picked by torch.randperm seeded with 0: the rows depend on the shape
+    alone, so two runs with the same arguments write the same rows."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: v.detach().float().cpu() for k, v in arrays.items()}
+    total = sum(v.numel() * 4 for v in arrays.values())
+    share = min(1.0, DUMP_BYTES / total) if total else 1.0
+    for name, v in arrays.items():
+        if share < 1.0:
+            n = max(1, int(v.shape[0] * share))
+            rows = torch.randperm(v.shape[0], generator=torch.Generator().manual_seed(0))[:n].sort().values
+            v = v[rows]
+        np.save(os.path.join(out_dir, name + ".npy"), v.numpy())
+
+
+def named_outputs(out):
+    """The engine's 10-tuple -> {output name: tensor} for the outputs the step computed (attention maps excluded)."""
+    from vilbert_b200 import _lib as L
+    return {k: v for k, v in zip(L.OUTPUT_FIELDS, out[:9]) if v is not None}
 
 
 class ClockSampler(threading.Thread):
@@ -322,7 +356,8 @@ def measure_vqa(args, model, reqs, dev, world, rank, local_rank, select, with_pr
     assert torch.allclose(chk, hout["vil_prediction"], atol=1e-5), "host/device C-ABI paths disagree"
 
     res = dict(value=value, ms=ms, per_rank_ms=per_rank, e2e_value=e2e_value, e2e_s=e2e_s, in_bytes=in_bytes, out_bytes=out_bytes,
-               n_launch=int(n_launch), flops=flops, nfl=nfl, enfl=enfl, clocks=sampler.result(), timed_region_s=ms * 1e-3)
+               n_launch=int(n_launch), flops=flops, nfl=nfl, enfl=enfl, clocks=sampler.result(), timed_region_s=ms * 1e-3,
+               last_out=named_outputs(out))
     if with_profile:
         # ---- per-kernel times, live: every kernel of the step replayed from its own CUDA graph between two CUDA events
         ops = model.profile_ops(B, Tin, V, select, iters=5)
@@ -373,6 +408,8 @@ def run_vqa(args):
 
     model = make_engine(args, sd, cfg, head, local_rank)
     m = measure_vqa(args, model, reqs, dev, world, rank, local_rank, select, with_profile=True)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, m["last_out"])
     par = parity_rows(model, oracle, reqs[0], rows) if rank == 0 else None
     weight_mb = model._dims["weight_bytes"] / 1e6
     model.close()
@@ -494,6 +531,8 @@ def run_multitask(args):
     ms_local, out, _ = timed_loop(step, args.steps, args.warmup, streams, dev, world, sampler)
     ms, per_rank = all_rank_ms(ms_local, world, dev)
     sampler.join(timeout=1.0)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, named_outputs(out))
     n_launch, flops = model.plan_info(hi - lo, Tin, V, select)
     # parity on this rank's slice: rows re-run alone must give the same bits (shard independence), rank 0 also checks the oracle
     o_all = model(*dreqs[0], select=select)
@@ -590,6 +629,8 @@ def run_retrieval(args):
     ms, per_rank = all_rank_ms(e0.elapsed_time(e1), world, dev)
     sampler.join(timeout=1.0)
     assert full.shape == (n_cap, n_img) and torch.isfinite(full).all()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"scores": full})
     # ---- checks on EVERY rank: (a) the gathered matrix is the same on all ranks, (b) sampled entries, recomputed here with the
     # plain full forward of that pair (no sharding, no reuse), match the matrix bit for bit; rank 0: (c) two entries vs the oracle
     csum = full.double().sum().reshape(1)

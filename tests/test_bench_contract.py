@@ -5,6 +5,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -40,3 +42,50 @@ def test_gpu_arm_fails_loudly_without_a_gpu():
     assert r.returncode != 0
     assert "no CPU fallback" in (r.stderr + r.stdout)
     assert not [l for l in r.stdout.splitlines() if l.startswith("{")]
+
+
+def test_dump_outputs_keeps_a_fixed_row_sample_within_the_budget(tmp_path, monkeypatch):
+    """Under the budget every output is written whole, as float32; over it every output keeps the same share of its rows, and
+    the same rows on every call, so dumps of two runs stay comparable."""
+    import numpy as np
+    import torch
+    import bench
+    a, b = torch.randn(100, 30, dtype=torch.float64), torch.randn(50, 4, 2)
+    bench.dump_outputs(str(tmp_path / "all"), {"a": a, "b": b})
+    whole = np.load(tmp_path / "all" / "a.npy")
+    assert whole.dtype == np.float32 and np.array_equal(whole, a.float().numpy())
+    monkeypatch.setattr(bench, "DUMP_BYTES", (a.numel() + b.numel()) * 4 // 4)
+    for d in ("s1", "s2"):
+        bench.dump_outputs(str(tmp_path / d), {"a": a, "b": b})
+    sa, sb = np.load(tmp_path / "s1" / "a.npy"), np.load(tmp_path / "s1" / "b.npy")
+    assert sa.shape == (25, 30) and sb.shape == (12, 4, 2)
+    assert sa.nbytes + sb.nbytes <= bench.DUMP_BYTES
+    assert np.array_equal(sa, np.load(tmp_path / "s2" / "a.npy")) and np.array_equal(sb, np.load(tmp_path / "s2" / "b.npy"))
+    rows = {tuple(r) for r in a.float().numpy()}
+    assert all(tuple(r) in rows for r in sa)
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_last_timed_step(tmp_path):
+    """--dump-outputs writes what the last of the --steps timed steps returned: 5 steps over 3 rotating input batches end on
+    batch (5 - 1) % 3 = 1, and a fresh engine given that batch returns the same bits."""
+    import numpy as np
+    import vilbert_b200 as vb
+    from vilbert_b200 import synthetic as S
+    out_dir = tmp_path / "dump"
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "5", "--warmup", "1", "--rotate", "3", "--batch", "8",
+                        "--dtype", "bf16", "--no-cpu-baseline", "--dump-outputs", str(out_dir)],
+                       capture_output=True, text=True, timeout=900, cwd=ROOT)
+    assert r.returncode == 0, r.stderr[-2000:]
+    line = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][-1])
+    assert line["steps"] == 5
+    assert sorted(os.listdir(out_dir)) == ["vil_prediction.npy"]
+    got = np.load(out_dir / "vil_prediction.npy")
+    assert got.dtype == np.float32 and got.shape == (8, 3129)
+    cfg = vb.BertConfig(task_specific_tokens=True, visualization=True)
+    model = vb.VILBertForVLTasks.from_pretrained(S.synthetic_state_dict(cfg, seed=42), config=cfg, num_labels=3129,
+                                                 compute_dtype="bf16").eval().cuda(0)
+    req = S.synthetic_request(8, 30, 36, seed=1234 + 1)
+    want = model(*[t.cuda() for t in req], select=vb.OUT_VIL_PREDICTION)[0].cpu().numpy()
+    model.close()
+    assert np.array_equal(got, want)

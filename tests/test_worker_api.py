@@ -265,9 +265,11 @@ def test_micro_batch_worker_close_cancels_queued_messages():
         late.result(timeout=5)
 
 
-def test_micro_batch_worker_round_trip():
+def test_micro_batch_worker_round_trip(monkeypatch):
     """Messages in the sender's schema (demo/sender.py:19-24) go in, WebSocket result dicts (worker.py:564-649) come out, and
-    concurrent messages share a model call."""
+    concurrent messages share a model call.  The stub computes on the CPU, so the worker is kept on its CPU path even where a
+    GPU is present (test_gpu_round2.py::test_micro_batch_worker_on_engine runs it on the engine)."""
+    monkeypatch.setattr(torch.cuda, "is_available", lambda: False)
     W.label_maps.update(vqa=None, gqa=None)
     W.model = RowModel()
     W.tokenizer = W.WordpieceTokenizer(VOCAB)
