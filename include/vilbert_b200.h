@@ -102,7 +102,9 @@ typedef struct {
     float* linguisic_prediction;   /* [B, T, vocab] */
     float* linguisic_logit;        /* [B, T, 1] */
     float* sequence_output_t;      /* optional debug tap: final text stream  [B, T, hidden]   (fp32) */
-    float* sequence_output_v;      /* optional debug tap: final image stream [B, V, v_hidden] (fp32) */
+    float* sequence_output_v;      /* optional debug tap: final image stream [B, V, v_hidden] (fp32).  Without a per-row head or
+                                      a sequence tap of a stream, its last layer (when it follows the last connection layer) runs
+                                      on row 0 of each sample only -- all the poolers read; asking for a tap keeps the full layer */
     float* pooled_output;          /* optional debug tap: pooled_t * pooled_v [B, bi_hidden] */
     float* attention_probs;        /* VB200_OUT_ATTENTION: one flat fp32 buffer holding every layer's softmax probabilities
                                       [B, heads, Lq, Lk] back to back in execution order (vb200_attention_layout gives the
@@ -177,7 +179,7 @@ int vb200_forward_host_slot(vb200_handle h, const vb200_inputs* in, const vb200_
                             int32_t synchronize, void* cuda_stream);
 
 /* Introspection used by the tests / bench: number of kernels one forward of this shape launches,
- * algorithmic FLOPs of it, model dimensions. */
+ * FLOPs it executes (a pruned tail counts its B-row work), model dimensions. */
 int vb200_plan_info(vb200_handle h, int32_t batch, int32_t n_tokens, int32_t n_regions, uint32_t select,
                     int64_t* n_launches, double* flops);
 int vb200_model_dim(vb200_handle h, const char* key, int64_t* value);
@@ -185,7 +187,9 @@ int vb200_model_dim(vb200_handle h, const char* key, int64_t* value);
  * GEMM with this percentage of the resident CTA slots as its persistent grid (production: two thirds, profiles/r2_grid_size.md) --
  * for reporting what a launch does when it has the GPU to itself; forwards are never affected.  "chain_ffn" (0/1): issue every
  * FFN-in -> FFN-out pair as ONE chained persistent launch (csrc/gemm_chain.cu: dynamic tile list + per-row-panel dependency counters;
- * same bits, measured slower at batch 64, profiles/r2_chain.md -> off by default); changing it drains the device and drops cached plans. */
+ * same bits, measured slower at batch 64, profiles/r2_chain.md -> off by default); changing it drains the device and drops cached plans.
+ * "prune_tail" (0/1, default 1, env VB200_PRUNE=0): run a stream's last layer after the last connection layer on the pooled rows only
+ * when no selected output reads that stream's sequence (same bits; for A/B runs); changing it drains the device and drops cached plans. */
 int vb200_set_option(vb200_handle h, const char* key, int64_t value);
 /* Profiling: after vb200_set_option(h, "timeline", 1) every tcgen05 GEMM launch of a forward records 16 stamps per CTA (0: clock64 at
  * entry, 1: setup done, 2: first k-block landed [-DVB200_STAMPS builds], 8 / 9: %globaltimer ns at entry / exit, 10: last MMA committed,

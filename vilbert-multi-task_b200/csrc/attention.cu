@@ -273,13 +273,15 @@ __device__ __forceinline__ void attend_tile_short(const uint16_t* Qs, const uint
 template <int D, bool F16>
 __global__ void __launch_bounds__(256, 2)     // <= 128 registers: 5 CTAs of 3-4 warps per SM -> one wave at batch 64
 self_attention_kernel(const uint16_t* __restrict__ qkv, int ld_qkv, int hidden, const float* __restrict__ key_mask_add,
-                      uint16_t* __restrict__ ctx, int ld_ctx, int L, float scale_l2, int pdl) {
+                      uint16_t* __restrict__ ctx, int ld_ctx, int L, int nq, float scale_l2, int pdl) {
+    // nq <= L: only the first nq query rows of each sample are computed (the last layer of a stream whose consumers read row 0
+    // alone); keys and values are always the sample's L rows, so a computed row has the same bits as in the full pass
     extern __shared__ __align__(16) uint8_t smem_attn[];
     constexpr int kStride = AttnTile<D>::kStride;
     const int h = blockIdx.x, b = blockIdx.y;
-    const int Lp = pad16(L);
+    const int Lp = pad16(L), Qp = pad16(nq);
     uint16_t* Qs = reinterpret_cast<uint16_t*>(smem_attn);
-    uint16_t* Ks = Qs + Lp * kStride;
+    uint16_t* Ks = Qs + Qp * kStride;
     uint16_t* Vs = Ks + Lp * kStride;
     float* mask_s = reinterpret_cast<float*>(Vs + Lp * kStride);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarps = blockDim.x >> 5;
@@ -287,7 +289,7 @@ self_attention_kernel(const uint16_t* __restrict__ qkv, int ld_qkv, int hidden, 
     if (pdl) pdl_wait();
 
     const uint16_t* base = qkv + static_cast<size_t>(b) * L * ld_qkv + h * D;
-    load_tile<D>(Qs, base, L, Lp, ld_qkv);
+    load_tile<D>(Qs, base, nq, Qp, ld_qkv);
     load_tile<D>(Ks, base + hidden, L, Lp, ld_qkv);
     load_tile<D>(Vs, base + 2 * hidden, L, Lp, ld_qkv);
     for (int j = threadIdx.x; j < L; j += blockDim.x) mask_s[j] = key_mask_add[b * L + j] * kLog2e;
@@ -297,12 +299,12 @@ self_attention_kernel(const uint16_t* __restrict__ qkv, int ld_qkv, int hidden, 
     uint16_t* outp = ctx + static_cast<size_t>(b) * L * ld_ctx + h * D;
     constexpr int kSplit = D / 64, kOW = D / kSplit;             // work item = (16-row tile, 64-column slice of the head)
     if (L <= kKeyBlock) {                                        // one key block: S and the softmax once per row tile
-        for (int t = warp; t * 16 < L; t += nwarps)
-            attend_tile_short<D, F16>(Qs, Ks, Vs, t * 16, L, L, mask_s, scale_l2, outp, ld_ctx, lane);
+        for (int t = warp; t * 16 < nq; t += nwarps)
+            attend_tile_short<D, F16>(Qs, Ks, Vs, t * 16, nq, L, mask_s, scale_l2, outp, ld_ctx, lane);
         return;
     }
-    for (int w = warp; (w / kSplit) * 16 < L; w += nwarps)
-        attend_tile<D, kOW, F16>(Qs, Ks, Vs, (w / kSplit) * 16, L, L, mask_s, scale_l2, outp, ld_ctx, lane, (w % kSplit) * kOW);
+    for (int w = warp; (w / kSplit) * 16 < nq; w += nwarps)
+        attend_tile<D, kOW, F16>(Qs, Ks, Vs, (w / kSplit) * 16, nq, L, mask_s, scale_l2, outp, ld_ctx, lane, (w % kSplit) * kOW);
 }
 
 template <int D, bool F16>
@@ -366,32 +368,31 @@ co_attention_kernel(const uint16_t* __restrict__ qkv_img, int ld_img, const uint
 
 template <int D, bool F16>
 static cudaError_t launch_self(const __nv_bfloat16* qkv, int ld_qkv, int hidden, const float* key_mask_add,
-                               __nv_bfloat16* ctx, int ld_ctx, int B, int L, int heads, int pdl, cudaStream_t st) {
-    const int Lp = pad16(L);
-    const size_t smem = 3 * AttnTile<D>::bytes(Lp) + sizeof(float) * L;
+                               __nv_bfloat16* ctx, int ld_ctx, int B, int L, int nq, int heads, int pdl, cudaStream_t st) {
+    const int Lp = pad16(L), Qp = pad16(nq);
+    const size_t smem = AttnTile<D>::bytes(Qp) + 2 * AttnTile<D>::bytes(Lp) + sizeof(float) * L;
     if (smem > 227 * 1024) return cudaErrorInvalidValue;
     cudaError_t e = set_smem(self_attention_kernel<D, F16>, smem);
     if (e != cudaSuccess) return e;
     static const int split_warps = [] { const char* e = getenv("VB200_ATTN_SPLIT_WARPS"); return e ? atoi(e) : 0; }();
     // one warp per 16-row tile, walking its D / 64 column slices in turn (measured better than one warp per slice: 3-warp CTAs
     // of the 128-wide heads fit five per SM -> one wave; VB200_ATTN_SPLIT_WARPS=1 for the other layout)
-    const int nwarps = min(8, (Lp / 16) * (split_warps ? D / 64 : 1));
+    const int nwarps = min(8, (Qp / 16) * (split_warps ? D / 64 : 1));
     const float scale_l2 = kLog2e / sqrtf(static_cast<float>(D));
     return launch_ex(self_attention_kernel<D, F16>, dim3(heads, B), dim3(32 * nwarps), smem, pdl, st,
                      reinterpret_cast<const uint16_t*>(qkv), ld_qkv, hidden, key_mask_add, reinterpret_cast<uint16_t*>(ctx),
-                     ld_ctx, L, scale_l2, pdl);
+                     ld_ctx, L, nq, scale_l2, pdl);
 }
 
 cudaError_t launch_self_attention(const __nv_bfloat16* qkv, int ld_qkv, int hidden, const float* key_mask_add,
-                                  __nv_bfloat16* ctx, int ld_ctx, int B, int L, int heads, int head_dim, int pdl,
+                                  __nv_bfloat16* ctx, int ld_ctx, int B, int L, int nq, int heads, int head_dim, int pdl,
                                   int f16, cudaStream_t st) {
-    if (L < 1 || (head_dim != 64 && head_dim != 128) || (ld_qkv & 7) || (ld_ctx & 1) || (hidden & 7))
+    if (L < 1 || nq < 1 || nq > L || (head_dim != 64 && head_dim != 128) || (ld_qkv & 7) || (ld_ctx & 1) || (hidden & 7))
         return cudaErrorInvalidValue;
-    if (head_dim == 64)
-        return f16 ? launch_self<64, true>(qkv, ld_qkv, hidden, key_mask_add, ctx, ld_ctx, B, L, heads, pdl, st)
-                   : launch_self<64, false>(qkv, ld_qkv, hidden, key_mask_add, ctx, ld_ctx, B, L, heads, pdl, st);
-    return f16 ? launch_self<128, true>(qkv, ld_qkv, hidden, key_mask_add, ctx, ld_ctx, B, L, heads, pdl, st)
-               : launch_self<128, false>(qkv, ld_qkv, hidden, key_mask_add, ctx, ld_ctx, B, L, heads, pdl, st);
+#define VB_SELF(D, F) launch_self<D, F>(qkv, ld_qkv, hidden, key_mask_add, ctx, ld_ctx, B, L, nq, heads, pdl, st)
+    if (head_dim == 64) return f16 ? VB_SELF(64, true) : VB_SELF(64, false);
+    return f16 ? VB_SELF(128, true) : VB_SELF(128, false);
+#undef VB_SELF
 }
 
 template <int D, bool F16>

@@ -377,7 +377,8 @@ struct Op {
     int ld_a = 0, ld_b = 0, hidden = 0;
     const float *mask_a = nullptr, *mask_b = nullptr;
     bf16 *ctx_a = nullptr, *ctx_b = nullptr;
-    int ld_ctx_a = 0, ld_ctx_b = 0, B = 0, La = 0, Lb = 0, heads = 0, head_dim = 0;
+    int ld_ctx_a = 0, ld_ctx_b = 0, B = 0, La = 0, Lb = 0, heads = 0, head_dim = 0;   // SELF_ATTN: Lb = query rows per sample
+                                                                                       //   when fewer than La (pruned tail), else 0
     // layernorm (un-fused): out = LN(ln_y + ln_res)
     const float *ln_y = nullptr, *ln_res = nullptr, *ln_g = nullptr, *ln_b = nullptr;
     float* ln_out_f = nullptr;
@@ -475,6 +476,8 @@ struct vb200_engine {
                                // (profiles/r2_b512.md): 2 waves when the GEMM has >= 20 row panels of 256 (batch >= ~160: 512: +5.7 %,
                                // 384: +2 %, 192: +1 %, 256: =), else 4 (batch 128 loses 4.5 % with 2).  VB200_PAIR_MIN_WAVES overrides.
     bool fused_ln = false;     // VB200_FUSED_LN=1: cluster-LayerNorm GEMM epilogue instead of GEMM(fp32) + row LayerNorm kernel
+    bool prune_tail = true;    // VB200_PRUNE=0 / vb200_set_option("prune_tail", 0): the last layer of a stream runs at full size even
+                               // when nothing reads its rows beyond row 0 of each sample (A/B runs; get_plan, tail_prunable)
     Arena weights;
     std::string last_error;
     // embeddings
@@ -1003,11 +1006,33 @@ struct vb200_engine {
     // the same rows, hence bit-identical scores.
     enum PlanMode { FULL = 0, TEXT_PREFIX = 1, IMAGE_PREFIX = 2, SUFFIX = 3 };
 
-    Plan* get_plan(int B, int Tin, int V, uint32_t select, int slot = 0, int mode = FULL, bool want_attn = false) {
+    // Pruned tail.  When a stream's last step is a single-stream layer after the last connection layer and nothing selected reads
+    // that stream's sequence (no per-row head, no sequence-output tap, no attention maps), the only reader of the layer's output is
+    // the pooler, which takes row 0 of each sample.  Then everything after the QKV projection (keys and values are still needed for
+    // every row) runs on those B rows alone.  Every kernel computes a row from that row alone in a fixed order, so the pooled
+    // outputs keep their bits.  Returns bit 0 for the text stream, bit 1 for the image stream.  seq_out: the same two bits for the
+    // sequence outputs the caller asks for.  The opt-in fp32-parity, LayerNorm-fold, fused-LayerNorm and chained-FFN modes keep the
+    // full tail.
+    int tail_prunable(uint32_t select, int mode, bool want_attn, int seq_out) const {
+        if (!prune_tail || x3 || ln_fold || fused_ln || chain_ffn || want_attn || mode == TEXT_PREFIX || mode == IMAGE_PREFIX) return 0;
+        int last_t = -1, last_v = -1, last_c = -1;
+        for (size_t i = 0; i < schedule.size(); ++i) {
+            const int k = static_cast<int>(i);
+            if (schedule[i][0] == 'T') last_t = k; else if (schedule[i][0] == 'V') last_v = k; else last_c = k;
+        }
+        int bits = 0;
+        if (last_t > last_c && !(seq_out & 1) && !(select & (VB200_OUT_LINGUISIC_PREDICTION | VB200_OUT_LINGUISIC_LOGIT))) bits |= 1;
+        if (last_v > last_c && !(seq_out & 2) && !(select & (VB200_OUT_VISION_PREDICTION | VB200_OUT_VISION_LOGIT))) bits |= 2;
+        return bits;
+    }
+
+    // seq_out: bit 0 / bit 1 = the caller reads the final text / image sequence (vb200_outputs::sequence_output_t / _v)
+    Plan* get_plan(int B, int Tin, int V, uint32_t select, int slot = 0, int mode = FULL, bool want_attn = false, int seq_out = 0) {
         if (slot < 0 || slot > 15) fail(VB200_ERR_INVALID, "slot %d out of range (0..15)", slot);
         if (slot > 0 && !opt.use_cuda_graph) fail(VB200_ERR_INVALID, "concurrent slots need CUDA-graph plans (use_cuda_graph)");
         if (mode == TEXT_PREFIX || mode == IMAGE_PREFIX) { select = 0; want_attn = false; }
-        std::vector<int64_t> key{B, Tin, V, static_cast<int64_t>(select), slot, mode, want_attn ? 1 : 0};
+        const int prune = tail_prunable(select, mode, want_attn, seq_out);
+        std::vector<int64_t> key{B, Tin, V, static_cast<int64_t>(select), slot, mode, want_attn ? 1 : 0, prune};
         auto it = plans.find(key);
         if (it != plans.end()) { it->second->last_use = ++use_clock; return it->second.get(); }
         std::unique_ptr<Plan> up(new Plan());
@@ -1074,14 +1099,15 @@ struct vb200_engine {
             return fa;
         };
         // GEMM + LayerNorm whose residual is buffers[rwhich] of stream st (its own LayerNorm possibly pending: res_pend);
-        // the result lands in buffers[owhich]; keep == true leaves THIS LayerNorm pending (statistics in stats[owhich])
-        auto ln_linear = [&](StreamSt& st, const bf16* A, int64_t lda, const LinearW& W, const LNW& ln, int rwhich, const LNW* res_pend,
-                             int owhich, bool keep, Op::Sync sync) {
+        // the result lands in buffers[owhich]; keep == true leaves THIS LayerNorm pending (statistics in stats[owhich]).
+        // M rows of A; the residual and the result are M rows of the stream buffers ld elements apart (pruned tail: row 0 of each sample)
+        auto ln_linear = [&](StreamSt& st, const bf16* A, int64_t M, int64_t lda, const LinearW& W, const LNW& ln, int rwhich,
+                             const LNW* res_pend, int owhich, bool keep, Op::Sync sync, int ld) {
             FoldArgs fa;
             fa.stats_ld = st.stats_ld;
             if (res_pend != nullptr) { fa.res_stats = st.stats[rwhich]; fa.res_parts = st.hid / 32; fa.res_ln = res_pend; }
             if (keep) fa.out_stats = st.stats[owhich];
-            add_linear(pl, A, st.rows, lda, W, vb::kActNone, st.f32[rwhich], st.hid, &ln, st.b16[owhich], st.hid, st.f32[owhich], st.hid,
+            add_linear(pl, A, M, lda, W, vb::kActNone, st.f32[rwhich], ld, &ln, st.b16[owhich], ld, st.f32[owhich], ld,
                        st.stream, sync, nullptr, 0, (res_pend != nullptr || keep) ? &fa : nullptr);
         };
 
@@ -1096,14 +1122,18 @@ struct vb200_engine {
         }
         if (do_v && ln_fold && fold_out_v.count("E") != 0) vs.pend = &vemb_ln;
 
-        // one BertLayer / BertImageLayer.  keep_out: this stage's output LayerNorm stays pending (LayerNorm fold map, ingest())
-        auto single_layer = [&](const LayerW& L, StreamSt& st, int inter, int heads, bool keep_out) {
-            const int hid = st.hid, cur = st.cur, M = st.rows, stream = st.stream;
+        // one BertLayer / BertImageLayer.  keep_out: this stage's output LayerNorm stays pending (LayerNorm fold map, ingest()).
+        // tail: pruned last layer of the stream (tail_prunable) -- QKV over every row, then attention, the output projection, the
+        // FFN and both LayerNorms for row 0 of each sample only, in place (rows b * seq of the stream buffers, row stride seq * hid;
+        // the FFN intermediate is compact [B, inter]).  The other rows of the stream buffers keep the layer's input.
+        auto single_layer = [&](const LayerW& L, StreamSt& st, int inter, int heads, bool keep_out, bool tail) {
+            const int hid = st.hid, cur = st.cur, stream = st.stream;
+            const int M = tail ? B : st.rows, ld = tail ? st.seq * hid : hid, nq = tail ? 1 : st.seq;
             bf16* qb; float* qf;
             qkv_out(st.qkv, qb, qf);
             {
                 FoldArgs fa = fold_in_args(st, cur);
-                add_linear(pl, st.b16[cur], M, hid, L.qkv, vb::kActNone, nullptr, 0, nullptr, qb, 3 * hid, qf, 3 * hid, stream, Op::NONE,
+                add_linear(pl, st.b16[cur], st.rows, hid, L.qkv, vb::kActNone, nullptr, 0, nullptr, qb, 3 * hid, qf, 3 * hid, stream, Op::NONE,
                            nullptr, 0, st.pend ? &fa : nullptr);
             }
             if (!x3) {
@@ -1111,8 +1141,8 @@ struct vb200_engine {
                 a.kind = Op::SELF_ATTN;
                 a.stream = stream;
                 a.qkv_a = qb; a.ld_a = 3 * hid; a.hidden = hid; a.mask_a = st.mask; a.ctx_a = st.ctx; a.ld_ctx_a = hid;
-                a.B = B; a.La = st.seq; a.heads = heads; a.head_dim = hid / heads;
-                a.flops = 4.0 * B * heads * st.seq * st.seq * (hid / heads);
+                a.B = B; a.La = st.seq; a.Lb = nq < st.seq ? nq : 0; a.heads = heads; a.head_dim = hid / heads;
+                a.flops = 4.0 * B * heads * nq * st.seq * (hid / heads);
                 pl.flops += a.flops;
                 ops.push_back(a);
             }
@@ -1120,20 +1150,25 @@ struct vb200_engine {
                 add_attn_f32(pl, qkv_at(st.qkv, 0), 3 * hid, qkv_at(st.qkv, hid), qkv_at(st.qkv, 2 * hid), 3 * hid, st.mask, st.seq, st.seq,
                              heads, hid, st.ctx, want_attn, stream);
             // attention output + LayerNorm1 (residual: the layer input) -> buffers [1 - cur]
-            ln_linear(st, st.ctx, hid, L.attn_out, L.ln1, cur, st.pend, 1 - cur, ln_fold, Op::NONE);
+            ln_linear(st, st.ctx, M, ld, L.attn_out, L.ln1, cur, st.pend, 1 - cur, ln_fold, Op::NONE, ld);
             {
                 FoldArgs fa = fold_in_args(st, 1 - cur);
-                add_linear(pl, st.b16[1 - cur], M, hid, L.inter, vb::kActGelu, nullptr, 0, nullptr, st.inter, inter, nullptr, 0, stream,
+                add_linear(pl, st.b16[1 - cur], M, ld, L.inter, vb::kActGelu, nullptr, 0, nullptr, st.inter, inter, nullptr, 0, stream,
                            Op::NONE, nullptr, 0, ln_fold ? &fa : nullptr);
             }
             // FFN output + LayerNorm2 (residual: LayerNorm1's output) -> buffers [cur]
-            ln_linear(st, st.inter, inter, L.out, L.ln2, 1 - cur, ln_fold ? &L.ln1 : nullptr, cur, keep_out, Op::NONE);
+            ln_linear(st, st.inter, M, inter, L.out, L.ln2, 1 - cur, ln_fold ? &L.ln1 : nullptr, cur, keep_out, Op::NONE, ld);
             st.pend = keep_out ? &L.ln2 : nullptr;
         };
 
         for (Op& op : ops) op.tag = "embed";
         bool in_suffix = false;
         size_t tagged = ops.size();
+        const std::string* tail_t = nullptr, *tail_v = nullptr;          // the layers tail_prunable prunes (last T / last V step)
+        for (const std::string& step : schedule) {
+            if (step[0] == 'T' && (prune & 1)) tail_t = &step;
+            if (step[0] == 'V' && (prune & 2)) tail_v = &step;
+        }
         for (const std::string& step : schedule) {
             for (; tagged < ops.size(); ++tagged) if (ops[tagged].tag == nullptr) ops[tagged].tag = "?";
             const int idx = atoi(step.c_str() + 1);
@@ -1143,9 +1178,11 @@ struct vb200_engine {
                 ~Tagger() { for (size_t i = from; i < ops.size(); ++i) ops[i].tag = name; }
             } tagger{ops, ops.size(), step.c_str()};
             if (step[0] == 'T') {
-                if (in_suffix ? do_s : do_t) single_layer(t_layers[idx], ts, c.inter, c.heads, ln_fold && fold_out_t.count(step) != 0);
+                if (in_suffix ? do_s : do_t)
+                    single_layer(t_layers[idx], ts, c.inter, c.heads, ln_fold && fold_out_t.count(step) != 0, &step == tail_t);
             } else if (step[0] == 'V') {
-                if (in_suffix ? do_s : do_v) single_layer(v_layers[idx], vs, c.v_inter, c.v_heads, ln_fold && fold_out_v.count(step) != 0);
+                if (in_suffix ? do_s : do_v)
+                    single_layer(v_layers[idx], vs, c.v_inter, c.v_heads, ln_fold && fold_out_v.count(step) != 0, &step == tail_v);
             } else if (do_s) {
                 const ConnW& W = c_layers[idx];
                 const int tcur = ts.cur, vcur = vs.cur;
@@ -1180,22 +1217,22 @@ struct vb200_engine {
                 ops[first_co].sync = Op::JOIN;              // needs both projections
                 const bool keep_v = ln_fold && fold_out_v.count(step) != 0, keep_t = ln_fold && fold_out_t.count(step) != 0;
                 // image branch (side stream; forks from the co-attention): biOutput.dense1 + LayerNorm1, v_intermediate, v_output + LayerNorm
-                ln_linear(vs, ctx_v, Hb, W.dense1, W.ln1, vcur, vs.pend, 1 - vcur, ln_fold, Op::FORK);
+                ln_linear(vs, ctx_v, Mv, Hb, W.dense1, W.ln1, vcur, vs.pend, 1 - vcur, ln_fold, Op::FORK, Hv);
                 {
                     FoldArgs fa = fold_in_args(vs, 1 - vcur);
                     add_linear(pl, pl.v_b16[1 - vcur], Mv, Hv, W.v_inter, vb::kActGelu, nullptr, 0, nullptr, inter_v, c.v_inter, nullptr, 0, 1,
                                Op::NONE, nullptr, 0, ln_fold ? &fa : nullptr);
                 }
-                ln_linear(vs, inter_v, c.v_inter, W.v_out, W.v_ln, 1 - vcur, ln_fold ? &W.ln1 : nullptr, vcur, keep_v, Op::NONE);
+                ln_linear(vs, inter_v, Mv, c.v_inter, W.v_out, W.v_ln, 1 - vcur, ln_fold ? &W.ln1 : nullptr, vcur, keep_v, Op::NONE, Hv);
                 vs.pend = keep_v ? &W.v_ln : nullptr;
                 // text branch (main stream)
-                ln_linear(ts, ctx_t, Hb, W.dense2, W.ln2, tcur, ts.pend, 1 - tcur, ln_fold, Op::NONE);
+                ln_linear(ts, ctx_t, Mt, Hb, W.dense2, W.ln2, tcur, ts.pend, 1 - tcur, ln_fold, Op::NONE, H);
                 {
                     FoldArgs fa = fold_in_args(ts, 1 - tcur);
                     add_linear(pl, pl.t_b16[1 - tcur], Mt, H, W.t_inter, vb::kActGelu, nullptr, 0, nullptr, inter_t, c.inter, nullptr, 0, 0,
                                Op::NONE, nullptr, 0, ln_fold ? &fa : nullptr);
                 }
-                ln_linear(ts, inter_t, c.inter, W.t_out, W.t_ln, 1 - tcur, ln_fold ? &W.ln2 : nullptr, tcur, keep_t, Op::NONE);
+                ln_linear(ts, inter_t, Mt, c.inter, W.t_out, W.t_ln, 1 - tcur, ln_fold ? &W.ln2 : nullptr, tcur, keep_t, Op::NONE, H);
                 ts.pend = keep_t ? &W.t_ln : nullptr;
             }
         }
@@ -1203,8 +1240,9 @@ struct vb200_engine {
         if ((do_s || do_v) && vs.pend != nullptr) fail(VB200_ERR_INVALID, "LayerNorm fold: the image stream ends with a pending LayerNorm");
         const int tc = ts.cur, vc = vs.cur;
         pl.t_cur = tc; pl.v_cur = vc;
-        pl.outs[9] = OutBuf{pl.t_f32[tc], Mt, H, H};
-        pl.outs[10] = OutBuf{pl.v_f32[vc], Mv, Hv, Hv};
+        // a pruned stream holds final values in row 0 of each sample only: its sequence output stays unavailable
+        if (!(prune & 1)) pl.outs[9] = OutBuf{pl.t_f32[tc], Mt, H, H};
+        if (!(prune & 2)) pl.outs[10] = OutBuf{pl.v_f32[vc], Mv, Hv, Hv};
 
         const size_t n_before_heads = ops.size();
         if (do_s) build_heads(pl, select);
@@ -1348,7 +1386,7 @@ struct vb200_engine {
                 break;
             case Op::SELF_ATTN:
                 CUDA_CHECK(vb::launch_self_attention(op.qkv_a, op.ld_a, op.hidden, op.mask_a, op.ctx_a, op.ld_ctx_a, op.B, op.La,
-                                                     op.heads, op.head_dim, light_pdl(), opt.act_fp16, st));
+                                                     op.Lb > 0 ? op.Lb : op.La, op.heads, op.head_dim, light_pdl(), opt.act_fp16, st));
                 break;
             case Op::CO_ATTN:
                 CUDA_CHECK(vb::launch_co_attention(op.qkv_a, op.ld_a, op.qkv_b, op.ld_b, op.hidden, op.mask_a, op.mask_b, op.ctx_a,
@@ -1587,6 +1625,9 @@ struct vb200_engine {
                                            c.v_hidden, c.v_hidden * S, st));
         run_plan(pl, st);
     }
+    static int seq_out(const vb200_outputs& o) {       // get_plan's seq_out bits for the sequence outputs the caller reads
+        return (o.sequence_output_t != nullptr ? 1 : 0) | (o.sequence_output_v != nullptr ? 2 : 0);
+    }
     static float* out_ptr(const vb200_outputs& o, int slot) {
         switch (slot) {
             case 0: return o.vil_prediction; case 1: return o.vil_prediction_gqa; case 2: return o.vil_logit;
@@ -1601,7 +1642,8 @@ struct vb200_engine {
             float* dst = out_ptr(out, s);
             const OutBuf& o = pl.outs[s];
             if (dst == nullptr) continue;
-            if (o.p == nullptr) fail(VB200_ERR_INVALID, "output slot %d requested but not selected in the `select` mask", s);
+            if (o.p == nullptr) fail(VB200_ERR_INVALID, "output slot %d requested but not %s", s,
+                                     s >= 9 && s <= 10 ? "available from this plan" : "selected in the `select` mask");
             CUDA_CHECK(cudaMemcpy2DAsync(dst, static_cast<size_t>(o.cols) * 4, o.p, static_cast<size_t>(o.ld) * 4,
                                          static_cast<size_t>(o.cols) * 4, o.rows, kind, st));
         }
@@ -1685,6 +1727,7 @@ int vb200_create(const char* config_json, int64_t n_tensors, const vb200_tensor*
         if (const char* v = getenv("VB200_TRI")) eng->tri_min_tiles = std::max(0, atoi(v));
         if (const char* v = getenv("VB200_LONE_ROWS")) eng->lone_rows = std::max(0, atoi(v));
         if (const char* v = getenv("VB200_CHAIN")) eng->chain_ffn = (strcmp(v, "0") != 0);
+        if (const char* v = getenv("VB200_PRUNE")) eng->prune_tail = (strcmp(v, "0") != 0);
         eng->ln_fold = o.ln_fold > 0;
         if (const char* v = getenv("VB200_LNFOLD")) eng->ln_fold = (strcmp(v, "0") != 0);
         if (eng->x3 || eng->fused_ln) eng->ln_fold = false;      // those modes keep every LayerNorm as its own step
@@ -1735,7 +1778,7 @@ int vb200_forward_slot(vb200_handle h, const vb200_inputs* in, const vb200_outpu
         if (in == nullptr || out == nullptr) fail(VB200_ERR_INVALID, "inputs/outputs struct is NULL");
         CUDA_CHECK(cudaSetDevice(h->opt.device));
         Plan* pl = h->get_plan(in->batch, in->n_tokens, in->n_regions, select & VB200_OUT_ALL, slot, vb200_engine::FULL,
-                               (select & VB200_OUT_ATTENTION) != 0);
+                               (select & VB200_OUT_ATTENTION) != 0, vb200_engine::seq_out(*out));
         cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
         h->forward_device(*pl, *in, st);
         h->copy_outputs(*pl, *out, st, cudaMemcpyDeviceToDevice);
@@ -1750,7 +1793,7 @@ int vb200_forward_regions(vb200_handle h, const vb200_region_inputs* in, const v
         if (in->n_boxes < 1) fail(VB200_ERR_INVALID, "n_boxes must be positive");
         CUDA_CHECK(cudaSetDevice(h->opt.device));
         Plan* pl = h->get_plan(in->batch, in->n_tokens, in->n_boxes + 1, select & VB200_OUT_ALL, slot, vb200_engine::FULL,
-                               (select & VB200_OUT_ATTENTION) != 0);
+                               (select & VB200_OUT_ATTENTION) != 0, vb200_engine::seq_out(*out));
         cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
         h->forward_regions(*pl, *in, st);
         h->copy_outputs(*pl, *out, st, cudaMemcpyDeviceToDevice);
@@ -1788,7 +1831,7 @@ int vb200_forward_cached(vb200_handle h, int32_t batch, int32_t n_tokens, int32_
         if (n_text < 1 || n_image < 1) fail(VB200_ERR_INVALID, "cached state counts must be positive");
         CUDA_CHECK(cudaSetDevice(h->opt.device));
         Plan* pl = h->get_plan(batch, n_tokens, n_regions, select & VB200_OUT_ALL, slot, vb200_engine::SUFFIX,
-                               (select & VB200_OUT_ATTENTION) != 0);
+                               (select & VB200_OUT_ATTENTION) != 0, vb200_engine::seq_out(*out));
         cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
         h->forward_cached(*pl, text_index, n_text, text_f32, text_16, text_mask, image_index, n_image, image_f32, image_16,
                           image_mask, st);
@@ -1834,7 +1877,7 @@ int vb200_forward_host_slot(vb200_handle h, const vb200_inputs* in, const vb200_
         if (in == nullptr || out == nullptr) fail(VB200_ERR_INVALID, "inputs/outputs struct is NULL");
         CUDA_CHECK(cudaSetDevice(h->opt.device));
         Plan* pl = h->get_plan(in->batch, in->n_tokens, in->n_regions, select & VB200_OUT_ALL, slot, vb200_engine::FULL,
-                               (select & VB200_OUT_ATTENTION) != 0);
+                               (select & VB200_OUT_ATTENTION) != 0, vb200_engine::seq_out(*out));
         cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
         const size_t B = pl->B, Tin = pl->Tin, V = pl->V, F = h->cfg.v_feat;
         if (pl->d_q == nullptr) {
@@ -1925,6 +1968,12 @@ int vb200_set_option(vb200_handle h, const char* key, int64_t value) {
                 CUDA_CHECK(cudaDeviceSynchronize());
                 h->plans.clear();
                 h->chain_ffn = value != 0;
+            }
+        } else if (k == "prune_tail") {
+            if ((value != 0) != h->prune_tail) {           // as chain_ffn: plans are built differently
+                CUDA_CHECK(cudaDeviceSynchronize());
+                h->plans.clear();
+                h->prune_tail = value != 0;
             }
         } else fail(VB200_ERR_INVALID, "unknown option \"%s\"", key);
     });
@@ -2093,7 +2142,7 @@ int vb200_self_attention(const void* qkv_bf16, int64_t ld_qkv, int32_t hidden, c
                          void* cuda_stream) {
     return op_guard([&] {
         CUDA_CHECK(vb::launch_self_attention(static_cast<const bf16*>(qkv_bf16), (int)ld_qkv, hidden, mask_add,
-                                             static_cast<bf16*>(ctx_bf16), (int)ld_ctx, B, L, heads, head_dim, 0,
+                                             static_cast<bf16*>(ctx_bf16), (int)ld_ctx, B, L, L, heads, head_dim, 0,
                                              act_fp16 ? 1 : 0, static_cast<cudaStream_t>(cuda_stream)));
     });
 }

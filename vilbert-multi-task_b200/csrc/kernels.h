@@ -69,9 +69,10 @@ cudaError_t launch_gemm_persistent_plain(const CUtensorMap& tmap_a, const CUtens
                                          int block_n, cudaStream_t st);
 
 // 16-bit activation buffers are typed __nv_bfloat16* throughout; `f16` says the bits are IEEE fp16 instead.
-// K4: softmax(Q K^T / sqrt(d) + mask) V per (sample, head); qkv row = [Q | K | V], each `hidden` wide.
+// K4: softmax(Q K^T / sqrt(d) + mask) V per (sample, head); qkv row = [Q | K | V], each `hidden` wide.  Context rows are
+// computed for the first nq (1..L) query rows of each sample, in place at rows b*L .. b*L + nq - 1 of ctx.
 cudaError_t launch_self_attention(const __nv_bfloat16* qkv, int ld_qkv, int hidden, const float* key_mask_add,
-                                  __nv_bfloat16* ctx, int ld_ctx, int B, int L, int heads, int head_dim, int pdl,
+                                  __nv_bfloat16* ctx, int ld_ctx, int B, int L, int nq, int heads, int head_dim, int pdl,
                                   int f16, cudaStream_t st);
 // K5: both co-attention directions in one kernel.  qkv_img rows = [Q1|K1|V1], qkv_txt rows = [Q2|K2|V2].
 //   ctx_txt[b,t] = softmax(Q2 K1^T / sqrt(d) + img_mask) V1      ctx_img[b,v] = softmax(Q1 K2^T / sqrt(d) + txt_mask) V2

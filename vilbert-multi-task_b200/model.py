@@ -197,7 +197,8 @@ class VILBertForVLTasks(object):
         return n.value, f.value
 
     def set_option(self, key, value):
-        """Run-time knobs of the engine (include/vilbert_b200.h, vb200_set_option): "max_plans", "chain_ffn", "profile_grid_pct"."""
+        """Run-time knobs of the engine (include/vilbert_b200.h, vb200_set_option): "max_plans", "chain_ffn", "prune_tail",
+        "profile_grid_pct"."""
         L.check(L.load().vb200_set_option(self._handle, key.encode(), int(value)), self._handle)
 
     def profile_ops(self, batch, n_tokens, n_regions, select=L.OUT_TASK_HEADS, iters=5, grid_pct=0):
